@@ -2,6 +2,7 @@
 """ehb200 benchmark — batched k-NN over the HNSW graph at the north-star configurations.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ehb200|reference] [--workload auto|c2|c3|...]
+                  [--dump-outputs DIR]
 
 Default workload ("auto"): ONE GPU -> BASELINE.json configs[2] (C3: N=10M d=768 Q=10k k=10 ef=128 InnerProduct,
 the north-star target, 30.7 GB of vectors on one B200); N > 1 GPUs -> configs[4] (C5: d=128 Q=10k k=100 ef=256
@@ -121,6 +122,16 @@ def shared_config(wl, world):
 def recall_at_k(found, truth):
     k = truth.shape[1]
     return float(np.mean([len(set(a.tolist()) & set(b.tolist())) / k for a, b in zip(found, truth)]))
+
+
+def dump_outputs(out_dir, labels, dists, counts):
+    """Writes the last timed step's result as <out_dir>/{labels,distances,counts}.npy so that two builds can be
+    compared output for output.  Labels go through int64 (NO_LABEL -> -1) to float64, exact below 2^53; the
+    largest workload (C5: Q=10k, k=100) writes about 12 MB, so every array is stored whole."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "labels.npy"), np.asarray(labels).view(np.int64).astype(np.float64))
+    np.save(os.path.join(out_dir, "distances.npy"), np.asarray(dists, dtype=np.float32))
+    np.save(os.path.join(out_dir, "counts.npy"), np.asarray(counts).astype(np.float32))
 
 
 class ClockSampler:
@@ -294,11 +305,21 @@ def run_reference(args, wl):
     if brute:
         ns, qs = min(N, 200_000), min(Q, 256)
         base = gen(ns, d, BASE_SEED)
-        best, med, passes = timed_passes(lambda: orc.bruteforce(base, q[:qs], k, wl["metric"], threads=cores), 3, 2, 60)
+        for _ in range(max(args.warmup, 1)):
+            orc.bruteforce(base, q[:qs], k, wl["metric"], threads=cores)
+        steps_ms = []
+        for _ in range(args.steps):
+            t0 = time.perf_counter()
+            labels, dists = orc.bruteforce(base, q[:qs], k, wl["metric"], threads=cores)
+            steps_ms.append((time.perf_counter() - t0) * 1e3)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, labels, dists, np.full(qs, min(k, ns)))
+        med = float(np.median(steps_ms)) * 1e-3
+        best = min(steps_ms) * 1e-3
         qps = qs / med * (ns / N)
         sample = (f"oracle exact scan of {qs} queries over the first {ns} base vectors on {cores} pinned threads, "
-                  f"scaled by {ns}/{N}; median of {passes} passes")
-        built, rec, t_build, steps_ms = ns, 1.0, 0.0, [med * 1e3]
+                  f"scaled by {ns}/{N}; median of {args.steps} steps")
+        built, rec, t_build = ns, 1.0, 0.0
     else:
         tune = {}
         o, base, t_build = oracle_build_prefix(orc, wl, args.ref_build_budget, cores, min(N, args.ref_max_points), tune)
@@ -317,8 +338,10 @@ def run_reference(args, wl):
         steps_ms = []
         for _ in range(args.steps):
             t0 = time.perf_counter()
-            labels, _, _ = o.search(qstep, k, ef=ef, threads=cores)
+            labels, dists, counts = o.search(qstep, k, ef=ef, threads=cores)
             steps_ms.append((time.perf_counter() - t0) * 1e3)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, labels, dists, counts)
         med = float(np.median(steps_ms)) * 1e-3
         best = min(steps_ms) * 1e-3
         gt, _ = orc.bruteforce(base, q[:200], k, wl["metric"], threads=cores)
@@ -467,6 +490,8 @@ def run_ehb(args, wl):
     st = counters[-1]
     kernel_name = ix.last_kernel_name()
     labels_dev = last["l"].cpu().numpy().view(np.uint64).copy()
+    if args.dump_outputs and rank == 0:     # every rank holds the same merged top-k
+        dump_outputs(args.dump_outputs, labels_dev, last["d"].cpu().numpy(), last["c"].cpu().numpy())
 
     # the local shard alone (no exchange), same steps: lets a reader separate the walk from the exchange
     shard_ms = None
@@ -710,7 +735,11 @@ def main():
     ap.add_argument("--ref-max-points", type=int, default=1_000_000)
     ap.add_argument("--recall-queries", type=int, default=2000)
     ap.add_argument("--dist", default="gaussian", choices=["gaussian", "gmm"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the labels, distances and counts of the last timed step to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     global DIST
     DIST = args.dist
     world = int(os.environ.get("WORLD_SIZE", str(args.gpus)))
